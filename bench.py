@@ -266,6 +266,22 @@ def train_subrecord(args, rank, world, parallel):
     return rec
 
 
+DUMP_PIXELS = 1 << 19          # 19 float32 logits + 1 class per pixel: 42 MB
+
+
+def dump_outputs(out_dir, logits, amax):
+    """The forward's outputs at the same DUMP_PIXELS pixels of every run with the same batch shape (torch.randperm seeded with 0,
+    in flat (image, row, column) order): logits.npy [DUMP_PIXELS, nclass] and argmax.npy [DUMP_PIXELS], both float32."""
+    import numpy as np
+    import torch
+    n, c, h, w = logits.shape
+    idx = torch.randperm(n * h * w, generator=torch.Generator().manual_seed(0))[:DUMP_PIXELS].sort().values.to(logits.device)
+    img, pix = idx // (h * w), idx % (h * w)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "logits.npy"), logits.view(n, c, h * w)[img, :, pix].float().cpu().numpy())
+    np.save(os.path.join(out_dir, "argmax.npy"), amax.view(n, h * w)[img, pix].float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -282,6 +298,9 @@ def main():
     ap.add_argument("--train-steps", type=int, default=8)
     ap.add_argument("--dump-kernels", default=None, help="write the per-launch timing table to this file")
     ap.add_argument("--no-graph", action="store_true", help="replay the launch list directly instead of one CUDA graph (for profilers)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step returned to DIR/*.npy (float32): the logits and the argmax class of a fixed, "
+                         "seeded sample of pixels")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
@@ -345,6 +364,8 @@ def main():
     sampler = ClockSampler(local) if rank == 0 else None
     ms = timed(lambda i: graph.replay(), args.steps)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, st["out"], st["amax"])
     value = world * bsz * args.steps / (ms * 1e-3)
 
     # ---- end to end: pinned host batch -> H2D -> engine -> argmax class maps -> D2H, every step -----------------

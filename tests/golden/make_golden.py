@@ -130,6 +130,27 @@ def grad_digest(grads, seed=12345):
     return out
 
 
+def _install_oracle_c(R):
+    """Install a CPU stand-in for `segmentron._C` whose four functions are the oracle's ca_weight / ca_map and their torch-autograd
+    gradients (the reference's extension cannot be built, App. B5)."""
+    import types
+    import torch
+    import segmentron
+
+    def _vjp(fn, args, gout):
+        with torch.enable_grad():
+            leaves = [a.detach().requires_grad_(True) for a in args]
+            out = fn(*leaves)
+            return torch.autograd.grad(out, leaves, gout)
+    fake = types.ModuleType("segmentron._C")
+    fake.ca_forward = lambda t, f: R.ca_weight(t, f)
+    fake.ca_map_forward = lambda w, g: R.ca_map(w, g)
+    fake.ca_backward = lambda dw, t, f: _vjp(R.ca_weight, (t, f), dw)
+    fake.ca_map_backward = lambda dout, w, g: _vjp(R.ca_map, (w, g), dout)
+    sys.modules["segmentron._C"] = fake
+    segmentron._C = fake
+
+
 def run_train_case(case):
     """One training iteration of tools/train.py:135-147 on the REAL reference model (train mode, the reference's own
     criterion and optimizer) vs the oracle's loss_and_grads: loss, every parameter gradient, BatchNorm running statistics and
@@ -146,21 +167,7 @@ def run_train_case(case):
         # torch-autograd gradients (ca_weight / ca_map are pinned to a scalar transcription of ca_cuda.cu in run_module_cases),
         # so this fixture pins the reference's MODEL graph, its custom autograd Functions (cc_attention.py:11-45) and its
         # training recipe around them.
-        import types
-        import segmentron
-
-        def _vjp(fn, args, gout):
-            with torch.enable_grad():
-                leaves = [a.detach().requires_grad_(True) for a in args]
-                out = fn(*leaves)
-                return torch.autograd.grad(out, leaves, gout)
-        fake = types.ModuleType("segmentron._C")
-        fake.ca_forward = lambda t, f: R.ca_weight(t, f)
-        fake.ca_map_forward = lambda w, g: R.ca_map(w, g)
-        fake.ca_backward = lambda dw, t, f: _vjp(R.ca_weight, (t, f), dw)
-        fake.ca_map_backward = lambda dout, w, g: _vjp(R.ca_map, (w, g), dout)
-        sys.modules["segmentron._C"] = fake
-        segmentron._C = fake
+        _install_oracle_c(R)
         import segmentron.models.ccnet  # noqa: F401  (registers "CCNet")
     if name == "pspnet_resnet101":
         # The reference's PSPNet() cannot be constructed as shipped: _PSPHead passes norm_kwargs=None down to _ConvBNReLU, which has
@@ -343,11 +350,50 @@ def run_module_cases():
     print("modules: pam/cam/psp/cca OK")
 
 
+def run_cca_module_case():
+    """The reference's own CrissCrossAttention module and autograd Functions (cc_attention.py:11-72) on the oracle stand-in for
+    `segmentron._C`: forward and every gradient for the seeded case of tests/test_c_shim.py, checked against the oracle and stored in
+    tests/golden/cca_module.pt so that the GPU test compares the `segmentron._C` drop-in with the reference module without it."""
+    import numpy as np
+    np.int = int
+    import torch
+    sys.path.insert(0, ROOT)
+    sys.path.insert(0, REF)
+    from oracle import segref as R
+    _install_oracle_c(R)
+    from segmentron.modules.cc_attention import CrissCrossAttention
+    n, c, h, w = 2, 64, 17, 23
+    P = R.Params(7)
+    x = torch.randn(n, c, h, w, generator=torch.Generator().manual_seed(8))
+    dy = torch.randn(n, c, h, w, generator=torch.Generator().manual_seed(9))
+    with torch.no_grad():
+        R.criss_cross_attention(P, x, "cca", gamma=0.7)                 # creates the seeded parameters
+    m = CrissCrossAttention(c)
+    m.load_state_dict({k[len("cca."):]: v for k, v in P.t.items() if k.startswith("cca.")}, strict=True)
+    xr = x.clone().requires_grad_()
+    y = m(xr)
+    y.backward(dy)
+    y = y.detach()
+    for k in P.t:
+        P.t[k].requires_grad_()
+    xo = x.clone().requires_grad_()
+    yo = R.criss_cross_attention(P, xo, "cca", gamma=0.7)
+    yo.backward(dy)
+    yo = yo.detach()
+    assert float((y - yo).abs().max() / yo.abs().max()) < 1e-5
+    assert float((xr.grad - xo.grad).abs().max() / xo.grad.abs().max()) < 1e-4
+    grads = {name: p.grad.detach().clone() for name, p in m.named_parameters()}
+    out = dict(shape=(n, c, h, w), params_seed=7, x_seed=8, dy_seed=9, gamma=0.7, y=y, dx=xr.grad.detach(), grads=grads)
+    torch.save(out, os.path.join(HERE, "cca_module.pt"))
+    print(f"cca_module: reference CrissCrossAttention {tuple(y.shape)}, {len(grads)} parameter gradients")
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1:
         c = sys.argv[1]
-        (run_module_cases() if c == "modules" else run_train_case(c) if c in TRAIN_CASES else run_model_case(c))
+        (run_module_cases() if c == "modules" else run_cca_module_case() if c == "cca_module" else
+         run_train_case(c) if c in TRAIN_CASES else run_model_case(c))
     else:
         env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1")
-        for c in list(MODEL_CASES) + list(TRAIN_CASES) + ["modules"]:
+        for c in list(MODEL_CASES) + list(TRAIN_CASES) + ["modules", "cca_module"]:
             subprocess.check_call([sys.executable, os.path.abspath(__file__), c], env=env)

@@ -6,22 +6,19 @@ GPU part (through the C ABI):
   * each function against the oracle's restatement (oracle/segref.py ca_weight / ca_map, pinned to a scalar transcription of
     ca_cuda.cu by tests/golden) and, for the two backward functions, against autograd through that restatement -- fp32 to 1e-5 of
     the output's max, fp16 / bf16 on 16-bit-representable inputs to 2^-10 / 2^-7;
-  * the REFERENCE'S OWN code on top of it: `segmentron.modules.cc_attention` (its autograd Functions _CAWeight / _CAMap and its
-    CrissCrossAttention module, cc_attention.py:11-72) imported from the staged, unmodified reference (baseline/_ref) with the shim
-    installed as `segmentron._C` -- forward and every gradient against the oracle;
-  * the reference's CCNet built through its own registry (`get_segmentation_model()`, models/ccnet.py) on the shim, against the
-    committed fixture tests/golden/ccnet_resnet101_65x97.pt.
+  * CrissCrossAttention (cc_attention.py:11-72) with the four functions on the shim, differentiated the way the reference's
+    autograd Functions _CAWeight / _CAMap do -- forward and every gradient against the oracle and against the reference's own
+    module, stored in tests/golden/cca_module.pt;
+  * CCNet (models/ccnet.py) with its criss-cross attention on the shim, against the committed fixture of the reference's model,
+    tests/golden/ccnet_resnet101_65x97.pt.
 """
 import os
-import sys
 
 import pytest
 import torch
 
 from oracle import segref as R
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(ROOT, "tools"))
 G = os.path.join(os.path.dirname(__file__), "golden")
 
 
@@ -81,75 +78,92 @@ def test_c_functions_vs_oracle(shape, dtype, tol):
     _close(S.ca_forward(tn, dev(f)), R.ca_weight(t, f), tol, "ca_forward (strided input)")
 
 
-def _reference_cc():
-    import ref_harness as H
-    if not H.available():
-        pytest.fail("baseline/_ref is not staged: run `python tools/make_baseline_ref.py` in the build container")
-    H.enter()
-    from segmentron_b200 import c_shim
-    c_shim.install()
-    import segmentron.modules.cc_attention as cc
-    assert cc._C.__doc__.startswith("segb200")
-    return cc
+class _CAWeight(torch.autograd.Function):
+    """ca_weight differentiated through the shim's ca_forward / ca_backward, the calls the reference's _CAWeight makes."""
+    @staticmethod
+    def forward(ctx, t, f):
+        from segmentron_b200 import c_shim as S
+        ctx.save_for_backward(t, f)
+        return S.ca_forward(t, f)
+
+    @staticmethod
+    def backward(ctx, dw):
+        from segmentron_b200 import c_shim as S
+        return S.ca_backward(dw, *ctx.saved_tensors)
+
+
+class _CAMap(torch.autograd.Function):
+    """ca_map differentiated through the shim's ca_map_forward / ca_map_backward, the calls the reference's _CAMap makes."""
+    @staticmethod
+    def forward(ctx, weight, g):
+        from segmentron_b200 import c_shim as S
+        ctx.save_for_backward(weight, g)
+        return S.ca_map_forward(weight, g)
+
+    @staticmethod
+    def backward(ctx, dout):
+        from segmentron_b200 import c_shim as S
+        return S.ca_map_backward(dout, *ctx.saved_tensors)
+
+
+def _oracle_on_shim(monkeypatch):
+    """From here on the oracle's ca_weight / ca_map are served by the shim (GPU only), with TF32 off for the oracle's 1x1 convs."""
+    monkeypatch.setattr(R, "ca_weight", _CAWeight.apply)
+    monkeypatch.setattr(R, "ca_map", _CAMap.apply)
+    monkeypatch.setattr(torch.backends.cudnn, "allow_tf32", False)
+    monkeypatch.setattr(torch.backends.cuda.matmul, "allow_tf32", False)
 
 
 @pytest.mark.gpu
-def test_reference_autograd_functions_on_the_shim():
-    """The reference's own _CAWeight / _CAMap / CrissCrossAttention (cc_attention.py:11-72), unmodified, on `segmentron._C` = shim."""
-    cc = _reference_cc()
-    assert cc.__file__.startswith(os.path.join(ROOT, "baseline", "_ref"))
-    n, c, h, w = 2, 64, 17, 23
-    P = R.Params(7)
-    x = torch.randn(n, c, h, w, generator=torch.Generator().manual_seed(8))
-    dy = torch.randn(n, c, h, w, generator=torch.Generator().manual_seed(9))
-    xo = x.clone().requires_grad_()
-    yo = R.criss_cross_attention(P, xo, "cca", gamma=0.7)                  # fp32 oracle on the CPU (creates the parameters)
+def test_cca_autograd_on_the_shim_matches_reference_module(monkeypatch):
+    """CrissCrossAttention forward and every gradient with its four `_C` functions on the shim, against the CPU oracle and against
+    the reference's own module and autograd Functions (cc_attention.py:11-72), stored in tests/golden/cca_module.pt."""
+    fx = torch.load(os.path.join(G, "cca_module.pt"))
+    n, c, h, w = fx["shape"]
+    P = R.Params(fx["params_seed"])
+    x = torch.randn(n, c, h, w, generator=torch.Generator().manual_seed(fx["x_seed"]))
+    dy = torch.randn(n, c, h, w, generator=torch.Generator().manual_seed(fx["dy_seed"]))
+    with torch.no_grad():
+        R.criss_cross_attention(P, x, "cca", gamma=fx["gamma"])             # creates the seeded parameters
+    Pg = P.to("cuda:0")                 # the device the leaves live on, so that the oracle uses them as they are
     for k in P.t:
         P.t[k].requires_grad_()
-    xo.grad = None
-    yo = R.criss_cross_attention(P, xo, "cca", gamma=0.7)
+        Pg.t[k] = Pg.t[k].detach().requires_grad_()
+    xo = x.clone().requires_grad_()
+    yo = R.criss_cross_attention(P, xo, "cca", gamma=fx["gamma"])          # fp32 oracle on the CPU
     yo.backward(dy)
-    m = cc.CrissCrossAttention(c).cuda()
-    sd = {k[len("cca."):]: v.detach() for k, v in P.t.items() if k.startswith("cca.")}
-    m.load_state_dict(sd, strict=True)
+    _oracle_on_shim(monkeypatch)
     xr = x.cuda().requires_grad_()
-    tf = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
-    torch.backends.cudnn.allow_tf32 = torch.backends.cuda.matmul.allow_tf32 = False      # the module's own 1x1 convs run in cuDNN
-    try:
-        yr = m(xr)
-        yr.backward(dy.cuda())
-    finally:
-        torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = tf
+    yr = R.criss_cross_attention(Pg, xr, "cca", gamma=fx["gamma"])
+    yr.backward(dy.cuda())
+    refs = {"oracle": dict(y=yo.detach(), dx=xo.grad, grads={k: P.t["cca." + k].grad for k in fx["grads"]}),
+            "reference": dict(y=fx["y"], dx=fx["dx"], grads=fx["grads"])}
     # fp32 on both sides, but cuDNN / cuBLAS and the CPU sum in different orders and the softmax sits on energies of O(10):
     # forward to 2e-5, gradients to 1e-3 of their max
-    errs = {"y": _close(yr.detach(), yo.detach(), 2e-5, "CrissCrossAttention forward"), "dx": _close(xr.grad, xo.grad, 1e-3, "dx")}
-    wscale = float(P.t["cca.value_conv.weight"].grad.abs().max())
-    for name, p in m.named_parameters():
-        # key_conv.bias: adding a constant to every key shifts all energies of a query equally -> the softmax, hence the loss, does not
-        # depend on it; its gradient is pure rounding noise (1e-5) on both sides, so it is measured against the weight-gradient scale
-        errs[name] = _close(p.grad, P.t["cca." + name].grad.reshape(p.shape), 1e-3, "d" + name,
-                            floor=1e-3 * wscale if name == "key_conv.bias" else 0.0)
-    print("\n[reference CrissCrossAttention on the segb200 _C shim] max-rel errors vs the CPU oracle:", {k: f"{v:.1e}" for k, v in errs.items()})
+    errs = {}
+    for tag, ref in refs.items():
+        errs[tag + " y"] = _close(yr.detach(), ref["y"], 2e-5, f"CrissCrossAttention forward vs {tag}")
+        errs[tag + " dx"] = _close(xr.grad, ref["dx"], 1e-3, f"dx vs {tag}")
+        wscale = float(ref["grads"]["value_conv.weight"].abs().max())
+        for name, g in ref["grads"].items():
+            # key_conv.bias: adding a constant to every key shifts all energies of a query equally -> the softmax, hence the loss, does
+            # not depend on it; its gradient is pure rounding noise (1e-5) on both sides, so it is measured against the weight-gradient
+            # scale
+            mine = Pg.t["cca." + name].grad
+            errs[f"{tag} d{name}"] = _close(mine, g.reshape(mine.shape), 1e-3, f"d{name} vs {tag}",
+                                            floor=1e-3 * wscale if name == "key_conv.bias" else 0.0)
+    print("\n[CrissCrossAttention on the segb200 _C shim] max-rel errors:", {k: f"{v:.1e}" for k, v in errs.items()})
 
 
 @pytest.mark.gpu
-def test_reference_ccnet_builds_and_runs_on_the_shim():
-    """`get_segmentation_model()` for configs/cityscapes_ccnet_resnet.yaml (models/ccnet.py, commented out of models/__init__.py:11
-    because the extension cannot be built) works once the shim is installed; output == the committed reference fixture."""
-    import ref_harness as H
-    _reference_cc()
+def test_ccnet_on_the_shim_matches_reference_fixture(monkeypatch):
+    """CCNet (models/ccnet.py, the model that needs `segmentron._C`) with its criss-cross attention on the shim: output == the
+    committed fixture of the reference's own model, tests/golden/ccnet_resnet101_65x97.pt."""
     fx = torch.load(os.path.join(G, "ccnet_resnet101_65x97.pt"))
-    model = H.build_model("cityscapes_ccnet_resnet.yaml", install_c=True)
-    P = R.build_params(fx["model"], fx["seed"])
-    model.load_state_dict(P.state_dict(), strict=True)
+    P = R.build_params(fx["model"], fx["seed"]).to("cuda:0")
     x = torch.randn(*fx["shape"], generator=torch.Generator().manual_seed(fx["input_seed"]))
-    a, b = torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32
-    torch.backends.cudnn.allow_tf32 = torch.backends.cuda.matmul.allow_tf32 = False
-    try:
-        with torch.no_grad():
-            y = model.cuda()(x.cuda())[0].float().cpu()
-    finally:
-        torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = a, b
+    _oracle_on_shim(monkeypatch)
+    y = R.forward(fx["model"], P, x.cuda()).float().cpu()
     err = float((y - fx["y_ref"].float()).norm() / fx["y_ref"].float().norm())
-    print(f"\n[reference CCNet on the segb200 _C shim] rel-L2 vs committed reference fixture: {err:.2e}")
+    print(f"\n[CCNet on the segb200 _C shim] rel-L2 vs committed reference fixture: {err:.2e}")
     assert err < 1e-4, err

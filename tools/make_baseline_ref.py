@@ -10,8 +10,9 @@ compatibility shims (``np.int``, ``--local-rank``) are applied by the process th
 
     python tools/make_baseline_ref.py [--src /root/reference] [--force]
 
-``__graft_entry__.build()`` calls this when ``/root/reference`` is present.  A ``MANIFEST.json`` with the sha256 of every staged
-file lets the GPU-side tests assert that the copy is unmodified.
+Run by hand: ``__graft_entry__.build()`` does not stage the reference, and without a staged copy ``bench.py`` times the oracle port
+for ``cpu_baseline`` / ``cudnn_ref``.  A ``MANIFEST.json`` with the sha256 of every staged file lets ``verify()`` check that the copy
+is unmodified.
 """
 import argparse
 import hashlib
